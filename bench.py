@@ -219,6 +219,61 @@ def workload(name, world):
                 chunk=chunk)
 
 
+def alignment_records(L, res, fields):
+    """the alignments of a result set as a numpy structured array over the library's memory (no copy), restricted
+    to `fields` of mgb_alignment_t; pointer fields read as uint64 addresses"""
+    from metagraph_b200._lib import mgb_alignment_t
+    types = dict(mgb_alignment_t._fields_)
+    dt = np.dtype({"names": list(fields),
+                   "formats": [np.uint64 if issubclass(types[f], ctypes._Pointer) else np.dtype(types[f]) for f in fields],
+                   "offsets": [getattr(mgb_alignment_t, f).offset for f in fields],
+                   "itemsize": ctypes.sizeof(mgb_alignment_t)})
+    n_aln = int(L.mgb_results_num_alignments(res))
+    if not n_aln:
+        return np.zeros(0, dt)
+    alns = L.mgb_results_alignments(res)
+    raw = (ctypes.c_char * (n_aln * dt.itemsize)).from_address(ctypes.addressof(alns.contents))
+    return np.frombuffer(raw, dtype=dt, count=n_aln)
+
+
+OUTPUT_FIELDS = ("read_index", "orientation", "score", "offset", "query_begin", "query_len", "num_nodes",
+                 "sequence_len", "num_cigar_ops")
+
+
+def output_arrays(L, res, max_rows=1 << 20, n_detail=4096):
+    """What a caller of mgb_align_batch receives, as float arrays for --dump-outputs: every scalar field of every
+    alignment (of a seeded sample of `max_rows` alignments when there are more), and for a seeded sample of
+    `n_detail` of those rows the CIGAR operations, the aligned sequence and the node path, flattened, each with an
+    offsets array. Values are exact in the float type used (float32 below 2**24, float64 for node ids). Node paths
+    are left out when the result set carries none (MGB_NODES_NONE), and no array is empty."""
+    rec = alignment_records(L, res, OUTPUT_FIELDS + ("nodes", "sequence", "cigar"))
+    rng = np.random.default_rng(0)
+    rows = np.arange(len(rec)) if len(rec) <= max_rows else np.sort(rng.choice(len(rec), max_rows, replace=False))
+    out = {"num_alignments": np.array([len(rec)], np.float64), "rows": rows.astype(np.float64)}
+    for f in OUTPUT_FIELDS:
+        out[f] = rec[f][rows].astype(np.float64 if f == "read_index" else np.float32)
+    detail = rows[np.sort(rng.choice(len(rows), min(n_detail, len(rows)), replace=False))]
+    cigar, seq, nodes = [], [], []
+    for r in detail:
+        a = rec[r]
+        cigar.append(np.frombuffer(ctypes.string_at(int(a["cigar"]), 4 * int(a["num_cigar_ops"])), np.uint32))
+        seq.append(np.frombuffer(ctypes.string_at(int(a["sequence"]), int(a["sequence_len"])), np.uint8))
+        nodes.append(np.frombuffer(ctypes.string_at(int(a["nodes"]), 8 * int(a["num_nodes"])), np.uint64)
+                     if a["nodes"] else np.zeros(0, np.uint64))
+    def flat(parts, dtype):
+        return np.concatenate(parts) if parts else np.zeros(0, dtype)
+    ops = flat(cigar, np.uint32)   # packed (length << 3 | operation)
+    out.update(detail_rows=detail.astype(np.float64), cigar_length=(ops >> 3).astype(np.float32),
+               cigar_op=(ops & 7).astype(np.float32), sequence=flat(seq, np.uint8).astype(np.float32))
+    variable = [("cigar", cigar), ("sequence", seq)]
+    if any(len(p) for p in nodes):
+        out["nodes"] = flat(nodes, np.uint64).astype(np.float64)
+        variable.append(("nodes", nodes))
+    for name, parts in variable:
+        out[name + "_offsets"] = np.cumsum([0] + [len(p) for p in parts]).astype(np.float64)
+    return {name: a for name, a in out.items() if a.size}
+
+
 def rank_reads(wl, genome, rank, world):
     if wl["error_rate"] == 0.0:
         return make_reads(genome, wl["n_rank"], 42 + rank)
@@ -233,7 +288,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default=os.environ.get("BENCH_CONFIG", "c2"), choices=["c2", "c3"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the alignments of the last timed step (rank 0's reads) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
 
     rank = env_int("RANK", 0)
     world = env_int("WORLD_SIZE", 1)
@@ -338,28 +397,23 @@ def main():
         if world > 1:
             dist.barrier()
 
-    from metagraph_b200._lib import mgb_alignment_t
     from metagraph_b200.sharding import ResultGather
-    aln_dtype = np.dtype({"names": ["read_index", "orientation", "score"], "formats": ["<u4", "u1", "<i4"],
-                          "offsets": [mgb_alignment_t.read_index.offset, mgb_alignment_t.orientation.offset,
-                                      mgb_alignment_t.score.offset], "itemsize": ctypes.sizeof(mgb_alignment_t)})
     L = aligner._L
     gatherer = ResultGather(L, dev) if world > 1 else None
     gather_ms = []
 
     def score_sum(res):
-        n_aln = int(L.mgb_results_num_alignments(res))
-        alns = L.mgb_results_alignments(res)
-        raw = (ctypes.c_char * (n_aln * ctypes.sizeof(mgb_alignment_t))).from_address(
-            ctypes.addressof(alns.contents)) if n_aln else b""
-        view = np.frombuffer(raw, dtype=aln_dtype, count=n_aln)
-        return n_aln, int(np.add.reduce(view["score"], dtype=np.int64))
+        view = alignment_records(L, res, ("score",))
+        return len(view), int(np.add.reduce(view["score"], dtype=np.int64))
 
-    def step(gather):
+    def step(gather, outputs=None):
         """one pass over this rank's reads; with `gather` every rank's result set goes to rank 0, which reads the
-        score of every alignment of the whole job (checksum); otherwise each rank reads its own"""
+        score of every alignment of the whole job (checksum); otherwise each rank reads its own. `outputs` (a dict)
+        receives output_arrays() of the result set."""
         res = aligner.align_batch_raw(buf, offsets)
         st = aligner.stats_of(res)
+        if outputs is not None:
+            outputs.update(output_arrays(L, res))
         if gather and gatherer is not None:
             tg = time.time()
             parts = gatherer.gather(res, rank * N)
@@ -387,7 +441,9 @@ def main():
     barrier()
     if rank == 0:
         sampler.start()
-    stats = [step(False) for _ in range(args.steps)]
+    # the output copy of the last step is host work after its kernels: the device timers do not see it
+    outputs = {} if args.dump_outputs and rank == 0 else None
+    stats = [step(False, outputs if s == args.steps - 1 else None) for s in range(args.steps)]
     barrier()
     # the same region with the exact-path shortcut switched off (every extension runs): what the roofline / GCUPS
     # lines describe, and the device-timed rate without the shortcut
@@ -512,6 +568,10 @@ def main():
                                               % (n, dt, CPU_SUFFIX_INDEX, max(1, host_threads // 4),
                                                  max(1, host_threads // 2), host_threads, used_threads)}
         print(json.dumps(line))
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

@@ -2,6 +2,7 @@
 (host-emulation build) and gather the results on rank 0; the gathered lines must equal the oracle's
 output for the unsharded batch."""
 import os
+import socket
 import subprocess
 import sys
 
@@ -50,8 +51,11 @@ def test_two_rank_sharding_gloo(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text("ROOT = %r\n" % ROOT + WORKER)
     env = dict(os.environ, MASTER_ADDR="127.0.0.1", OMP_NUM_THREADS="1")
+    with socket.socket() as s:   # a free port: other jobs on the host may hold any fixed one
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
     out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-                          "--master-addr", "127.0.0.1", "--master-port", "29517", str(script)],
+                          "--master-addr", "127.0.0.1", "--master-port", str(port), str(script)],
                          capture_output=True, text=True, env=env, timeout=600)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-3000:]
     assert "SHARDING_OK 37" in out.stdout
